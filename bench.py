@@ -2,7 +2,7 @@
 """bench.py -- disvae training hot path on B200 (contract: see the task statement / DESIGN.md section 6).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-cuda]
-                  [--workload c1..c5] [--scaling weak|strong]
+                  [--workload c1..c5] [--scaling weak|strong] [--dump-outputs DIR]
 
 One "step" = one full optimisation step (forward, loss, backward, gradient all-reduce for N>1, Adam) over one
 synthetic batch.  Default workload at every N: BASELINE.json configs[1] (btcvae, 1x64x64, batch 1024 PER GPU, z=10,
@@ -16,7 +16,7 @@ bernoulli, MSS, Adam lr 5e-4) -- weak scaling.  `--scaling strong` divides the c
   ddp_parity (N>1): rank r's loss == oracle on shard r, rank-averaged gradients == mean of the oracle's shard gradients
   roofline / roofline_logdensity / cpu_baseline / cuda_eager_baseline / clocks / gpu_launches : DESIGN.md section 6
 
---impl reference      : the UNMODIFIED reference (baseline/_ref, shipped by scripts/ship_reference.py) through its own
+--impl reference      : the UNMODIFIED reference (oracle/_ref, shipped by oracle/ship_reference.py) through its own
                         Trainer._train_iteration on the host cores (kind "reference"); the oracle port if the copy is
                         not there (kind "port").
 --impl reference-cuda : the same unmodified reference with device=cuda (stock PyTorch eager: cuDNN/cuBLAS, TF32 off) --
@@ -136,6 +136,29 @@ class ClockSampler:
         return dict(sm_mhz=load[len(load) // 2], sm_max_mhz=mx, reasons=sorted(reasons), samples=len(sm))
 
 
+def dump_outputs(out_dir, trainer, loss):
+    """What the last timed step handed its caller, as DIR/<name>.npy (float32): the loss it returned and, updated in
+    place, every parameter and its gradient (the discriminator's too for FactorVAE).  Inputs, weights and noise are
+    seeded, so two builds run with the same arguments can be compared array for array.  At most 36 MB (c4: FactorVAE
+    with its discriminator's parameters and gradients); the assertion keeps it within 64 MB."""
+    import numpy as np
+    arrays = {"loss": loss}
+    nets = [("", trainer.model)]
+    if getattr(trainer.loss_f, "discriminator", None) is not None:
+        nets.append(("disc.", trainer.loss_f.discriminator))
+    for prefix, net in nets:
+        for k, p in net.named_parameters():
+            arrays["param." + prefix + k] = p
+            if p.grad is not None:
+                arrays["grad." + prefix + k] = p.grad
+    arrays = {k: t.detach().float().cpu().numpy() for k, t in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 * 1024 * 1024, "outputs to dump take %d bytes" % total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # =====================================================================================================
 # our arm
 # =====================================================================================================
@@ -190,14 +213,17 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}
+
     def timed(fn, n):
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(n):
-            fn(i)
+            r = fn(i)
         e1.record()
         barrier()
+        last["out"] = r
         ms = torch.tensor([e0.elapsed_time(e1)], device=device)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -219,6 +245,9 @@ def run_ours(args):
     ms = timed(step_res, K)
     launches = _native.launch_count() - l0
     clocks = clk.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # before the end-to-end and parity passes below move the model on (and replays overwrite the graph's loss)
+        dump_outputs(args.dump_outputs, trainer, last["out"])
     # untimed warm-up of the end-to-end path: three loader steps, and one EAGER step -- torch.cuda.graph empties the
     # caching allocator when it captures, so the first eager step afterwards (the every-50th logging step of a real
     # run) would otherwise pay ~2 GB of cudaMalloc inside the timed epoch, once
@@ -582,7 +611,7 @@ def oracle_job(workload, batch):
 
 def reference_job(workload, batch, device):
     """The unmodified reference's own training step: disvae.Trainer._train_iteration (training.py:137-164) of
-    baseline/_ref.  None if the copy is not there."""
+    oracle/_ref.  None if the copy is not there."""
     from oracle import reference_env
     ref = reference_env.find_reference()
     if ref is None:
@@ -664,7 +693,7 @@ def run_reference(args):
         step()
     dt = time.perf_counter() - t0
     v = round(Bs * args.steps / dt, 1)
-    what = ("unmodified reference (baseline/_ref) disvae.Trainer._train_iteration on CPU" if kind == "reference"
+    what = ("unmodified reference (oracle/_ref) disvae.Trainer._train_iteration on CPU" if kind == "reference"
             else "oracle port (oracle/disvae_oracle.py) on CPU")
     out = {"impl": "reference", "metric": "images/sec", "value": v, "unit": "img/s", "n_gpus": world, "steps": args.steps,
            "warmup": args.warmup, "ms_per_step": round(dt / args.steps * 1e3, 3), "higher_is_better": True,
@@ -695,7 +724,7 @@ def run_reference_cuda(args):
     B = per_gpu_batch(args, world)
     step = reference_job(args.workload, B, device)
     if step is None:
-        print(json.dumps({"impl": "reference-cuda", "unavailable": "baseline/_ref not shipped"}), flush=True)
+        print(json.dumps({"impl": "reference-cuda", "unavailable": "oracle/_ref not shipped"}), flush=True)
         return
     for _ in range(max(args.warmup, 3)):
         step()
@@ -712,7 +741,7 @@ def run_reference_cuda(args):
            "warmup": max(args.warmup, 3), "ms_per_step": round(ms / args.steps, 4), "higher_is_better": True,
            "scaling": args.scaling, "vs_baseline": None, "dtype": "f32", "data": "synthetic (torch.rand); random-init weights",
            "config": config_block(args, 1, B),
-           "what": "unmodified reference (baseline/_ref) disvae.Trainer._train_iteration, device=cuda, stock PyTorch %s eager "
+           "what": "unmodified reference (oracle/_ref) disvae.Trainer._train_iteration, device=cuda, stock PyTorch %s eager "
                    "(cuDNN %s), allow_tf32=False, cudnn.benchmark=True, batches resident" % (
                        torch.__version__, torch.backends.cudnn.version())}
     print(json.dumps(out), flush=True)
@@ -731,7 +760,14 @@ def main():
     ap.add_argument("--no-eager-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--detail", action="store_true", help="per-entry-point table on stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss, parameters and gradients of the last timed step to DIR/<name>.npy "
+                         "(--impl ours only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     elif args.impl == "reference-cuda":

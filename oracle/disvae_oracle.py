@@ -9,8 +9,8 @@ legs use it.
 
 Pinning status: the reference ships no tests or golden vectors for this path
 (SURVEY.md section 4), so the oracle is pinned against OUTPUTS OF THE REFERENCE
-ITSELF: `tests/golden/make_golden.py` imports the unmodified reference from
-/root/reference in the build container, runs it on seeded inputs and commits
+ITSELF: `tests/golden/make_golden.py` imports the unmodified reference from a
+checkout of it, runs it on seeded inputs and commits
 the results under `tests/golden/*.pt`; `tests/test_oracle_golden.py` checks
 every function below against those files.
 

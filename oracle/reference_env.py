@@ -1,5 +1,5 @@
-"""Import environment for the UNMODIFIED reference (baseline/_ref, shipped by scripts/ship_reference.py, or
-/root/reference in the build container).  TEST / BENCH INFRASTRUCTURE ONLY -- nothing under
+"""Import environment for the UNMODIFIED reference (git-ignored oracle/_ref, shipped by oracle/ship_reference.py
+during build()).  TEST / BENCH INFRASTRUCTURE ONLY -- nothing under
 `disentangling-vae_b200/` imports this.
 
 Two kinds of shim, neither touching arithmetic (SURVEY.md section 8c, Appendix C):
@@ -13,7 +13,7 @@ import sys
 import types
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CANDIDATES = [os.path.join(ROOT, "baseline", "_ref"), "/root/reference"]
+CANDIDATES = [os.path.join(ROOT, "oracle", "_ref")]
 
 
 def find_reference():
@@ -51,8 +51,8 @@ def activate(ref_dir=None, package_first=None):
     `disvae` is the one imported.  Returns the reference directory."""
     ref_dir = ref_dir or find_reference()
     if ref_dir is None:
-        raise RuntimeError("reference not found (expected baseline/_ref: run scripts/ship_reference.py in the build "
-                           "container)")
+        raise RuntimeError("reference not found (expected oracle/_ref: run oracle/ship_reference.py, or build(), "
+                           "where a checkout of the reference is available)")
     sys.dont_write_bytecode = True
     install_stubs()
     for d in (ref_dir, package_first):

@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """Generate the golden fixtures in tests/golden/ from the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference, which does not exist on
-the GPU box):
+Needs a checkout of the reference, found as build() finds it
+(oracle/ship_reference.py: $DISVAE_REFERENCE, BASELINE.json reference_path, or
+a directory named `reference` next to this repository):
 
     python tests/golden/make_golden.py
 
@@ -23,8 +24,12 @@ import sys
 import types
 from collections import defaultdict
 
-REF = os.environ.get("DISVAE_REFERENCE", "/root/reference")
 HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+from oracle.ship_reference import find_checkout  # noqa: E402
+
+REF = find_checkout()
+assert REF is not None, "no checkout of the reference found"
 
 sys.dont_write_bytecode = True
 sys.path.insert(0, REF)

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Child process of tests/test_main_gpu.py: the reference's UNMODIFIED `main.py` (baseline/_ref) drives THIS
-repository's `disvae` package on cuda:0 -- the proof of the drop-in boundary (SURVEY.md 8b, /root/reference
+"""Child process of tests/test_main_gpu.py: the reference's UNMODIFIED `main.py` (oracle/_ref) drives THIS
+repository's `disvae` package on cuda:0 -- the proof of the drop-in boundary (SURVEY.md 8b, reference
 main.py:165-247).  Only the data loader is replaced (there are no datasets on the box): `main.get_dataloaders` is
 looked up in main's globals (main.py:197,233), so assigning it is an injection, not a source edit.
 

@@ -228,7 +228,7 @@ def test_flat_grad_allreduce_world2_gloo(tmp_path):
 
 
 def test_bench_reference_arm_contract():
-    """`bench.py --impl reference` runs without a GPU (it times the unmodified reference shipped to baseline/_ref, or
+    """`bench.py --impl reference` runs without a GPU (it times the unmodified reference shipped to oracle/_ref, or
     the CPU oracle port when that copy is absent) and prints ONE JSON line with the keys the bench contract names; its
     metric/unit/config match our own arm's."""
     import json
@@ -245,7 +245,7 @@ def test_bench_reference_arm_contract():
     for k in ("value", "n_gpus", "steps", "warmup", "ms_per_step", "scaling", "vs_baseline", "dtype", "data", "config",
               "cpu_baseline", "e2e"):
         assert k in d, k
-    shipped = os.path.isfile(os.path.join(root, "baseline", "_ref", "main.py")) or os.path.isdir("/root/reference")
+    shipped = os.path.isfile(os.path.join(root, "oracle", "_ref", "main.py"))
     assert d["cpu_baseline"]["kind"] == ("reference" if shipped else "port") and d["cpu_baseline"]["value"] == d["value"]
     assert set(d["config"]) == {"workload", "loss", "img_size", "batch_per_gpu", "global_batch", "latent_dim", "n_data",
                                 "rec_dist", "optimizer", "parallelism", "l2"}          # == our own arm's keys

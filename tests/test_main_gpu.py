@@ -1,7 +1,7 @@
 """Drop-in boundary on hardware (SURVEY.md 8b): the reference's UNMODIFIED main.py (shipped to git-ignored
-baseline/_ref by scripts/ship_reference.py) trains, checkpoints, reloads and evaluates THIS repository's `disvae`
-package on the B200, then the reference's own visualiser decodes traversals through it
-(/root/reference main.py:165-247, utils/visualize.py:121-123,217-222).  Runs in a child process so that the
+oracle/_ref by oracle/ship_reference.py during build()) trains, checkpoints, reloads and evaluates THIS repository's
+`disvae` package on the B200, then the reference's own visualiser decodes traversals through it
+(reference main.py:165-247, utils/visualize.py:121-123,217-222).  Runs in a child process so that the
 reference's `main`/`utils` modules and the synthetic loader never leak into the other tests."""
 import json
 import os
@@ -13,13 +13,13 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "baseline", "_ref")
+REF = os.path.join(ROOT, "oracle", "_ref")
 
 
 @pytest.mark.parametrize("loss", ["btcvae", "factor"])
 def test_unmodified_main_drives_this_package(loss, tmp_path):
     if not os.path.isfile(os.path.join(REF, "main.py")):
-        pytest.skip("baseline/_ref not shipped (scripts/ship_reference.py runs in the build container)")
+        pytest.skip("oracle/_ref not shipped: build() found no checkout of the reference")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "run_reference_main.py"), loss, str(tmp_path)],
                        capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stdout[-3000:] + "\n" + r.stderr[-6000:]

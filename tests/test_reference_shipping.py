@@ -1,34 +1,39 @@
-"""baseline/_ref must be the reference byte for byte (CPU test; only meaningful in the build container where
-/root/reference exists)."""
-import filecmp
+"""oracle/_ref must be the reference byte for byte: every shipped source file against the SHA-256 digests of the
+original's files (tests/golden/reference_sha256.json, taken from YannDubs/disentangling-vae @ f0452191), and the copy
+must import as the reference's own `disvae` package.  CPU tests; they need the copy that build() ships when a checkout
+of the reference is available (oracle/ship_reference.py)."""
+import hashlib
+import json
 import os
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SRC, DST = "/root/reference", os.path.join(ROOT, "baseline", "_ref")
+DST = os.path.join(ROOT, "oracle", "_ref")
+DIGESTS = os.path.join(ROOT, "tests", "golden", "reference_sha256.json")
+
+
+def _need_copy():
+    if not os.path.isfile(os.path.join(DST, "main.py")):
+        pytest.skip("oracle/_ref not shipped: build() found no checkout of the reference")
 
 
 def test_shipped_reference_is_unmodified():
-    if not os.path.isdir(SRC) or not os.path.isdir(DST):
-        pytest.skip("needs /root/reference and baseline/_ref")
-    n = 0
+    _need_copy()
+    want = json.load(open(DIGESTS))
+    shipped = set()
     for base in ("disvae", "utils"):
-        for d, _, files in os.walk(os.path.join(SRC, base)):
-            for f in files:
-                if f.endswith(".py"):
-                    a = os.path.join(d, f)
-                    b = os.path.join(DST, os.path.relpath(a, SRC))
-                    assert filecmp.cmp(a, b, shallow=False), b
-                    n += 1
-    for f in ("main.py", "main_viz.py", "hyperparam.ini"):
-        assert filecmp.cmp(os.path.join(SRC, f), os.path.join(DST, f), shallow=False), f
-    assert n > 15
+        for d, _, files in os.walk(os.path.join(DST, base)):
+            shipped.update(os.path.relpath(os.path.join(d, f), DST) for f in files if f.endswith(".py"))
+    assert shipped == {k for k in want if k.startswith(("disvae/", "utils/"))}
+    for rel, digest in want.items():
+        with open(os.path.join(DST, rel), "rb") as fh:
+            assert hashlib.sha256(fh.read()).hexdigest() == digest, rel
+    assert len(want) > 15
 
 
 def test_reference_imports_from_shipped_copy():
-    if not os.path.isdir(DST):
-        pytest.skip("baseline/_ref not shipped")
+    _need_copy()
     import subprocess
     import sys
     code = ("import sys; sys.path.insert(0, %r); from oracle import reference_env as E; d = E.activate(%r); "
